@@ -504,6 +504,24 @@ def stats_of(ts):
     return dict(mean=float(a.mean()), median=float(np.median(a)), min=float(a.min()), max=float(a.max()))
 
 
+DUMP_SAMPLE = 1 << 20
+
+
+def step_outputs(model, rendered, loss):
+    """what a caller of the step receives, as float32 host arrays: the rendered buffers, the loss and every parameter's gradient (a fixed
+    seeded sample of DUMP_SAMPLE entries of a larger one, so that the whole dump stays far below 64 MB)"""
+    out = {f"rendered.{k}": v for k, v in rendered.items() if torch.is_tensor(v) and v.is_floating_point()}
+    out["loss"] = loss
+    for name, p in model.named_parameters():
+        if p.requires_grad and p.grad is not None:
+            g = p.grad.reshape(-1)
+            if g.numel() > DUMP_SAMPLE:
+                idx = np.sort(np.random.default_rng(0).choice(g.numel(), DUMP_SAMPLE, replace=False))
+                g = g[torch.from_numpy(idx).to(g.device)]
+            out[f"grad.{name}"] = g
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -525,7 +543,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-cuda", action="store_true")
     ap.add_argument("--dump-render", default=None, help="(internal) save the rendered buffers of view 0 to this file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="cfg2 only: after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32): the rendered "
+                         "buffers, the loss and the gradient of every parameter (of a parameter with more than 2^20 entries, a fixed seeded "
+                         "sample of 2^20 of them, in increasing index order)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl == "reference" or args.workload != "cfg2"):
+        ap.error("--dump-outputs is implemented for the cfg2 workload of the GPU arms")
 
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -624,7 +650,7 @@ def main():
             loss = total
         if world > 1:
             dist.all_reduce(flat)                # the one collective of a step: sum of the flat gradient
-        last["rendered"] = rendered
+        last["rendered"], last["loss"] = rendered, loss
         return loss
 
     def timed(fn, k, sampler=None):
@@ -673,6 +699,8 @@ def main():
         torch.cuda.synchronize()
         t_res = timed(resident, args.steps, clocks)      # ... and the one clock query comes after its last launch (see ClockSampler)
         gc.enable()
+        # the instrumented pass below reuses these buffers: keep what the last timed step computed
+        timed_out = step_outputs(model, last["rendered"], last["loss"]) if args.dump_outputs else None
         overflow = int(frame.counts()["overflow"]) if frame is not None else 0
         # a separate, instrumented pass for the roofline: the same step launched kernel by kernel with CUDA events around every launch of
         # the hash-gather kernels (not part of `value`); sizes are read back after every step to count the points that were processed
@@ -723,6 +751,10 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if timed_out is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in timed_out.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
 
     peaks = {}
     try:

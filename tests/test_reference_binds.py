@@ -1,25 +1,16 @@
-"""The drop-in boundary from the reference's side: an UNMODIFIED nr3d_lib Python tree imports and binds over
-`install_as_nr3d_lib_bindings()` (SURVEY.md §8b: "all of these names must resolve").  Needs /root/reference (the build container);
-the reference's package __init__ files pull uninstallable dependencies (addict, kornia, imageio ...), so -- as tests/golden/make_golden.py --
-the parent packages are registered empty with the right __path__ and the reference FILES are executed verbatim."""
+"""The drop-in boundary from the reference's side: what an UNMODIFIED nr3d_lib Python tree imports from and calls on
+`nr3d_lib.bindings` resolves over `install_as_nr3d_lib_bindings()` (SURVEY.md §8b: "all of these names must resolve").  What the reference's
+files import and call, and what its `LoTD` module built over the shim, are recorded in tests/golden/ref_binds.json by
+tests/golden/make_ref_binds.py from the reference tree."""
 import importlib
+import json
 import os
-import re
 import sys
 import types
 
 import pytest
-import torch
 
-REF = "/root/reference/nr3d_lib/nr3d_lib"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree only exists in the build container")
-
-
-def _pkg(name, path):
-    m = types.ModuleType(name)
-    m.__path__ = [path]
-    sys.modules[name] = m
-    return m
+GOLDEN = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_binds.json")))
 
 
 @pytest.fixture(scope="module")
@@ -28,15 +19,10 @@ def ref_tree():
     for k in saved:
         del sys.modules[k]
     import neuralsim_b200.bindings as B
-    _pkg("nr3d_lib", REF)
-    for sub in ("graphics", "graphics/pack_ops", "models", "models/grid_encodings", "models/grid_encodings/lotd", "models/embedders",
-                "models/embedders/spherical_harmonics", "models/spatial", "models/grid_encodings/permuto", "models/embedders/sinusoidal_cuda"):
-        _pkg("nr3d_lib." + sub.replace("/", "."), f"{REF}/{sub}")
+    root = types.ModuleType("nr3d_lib")
+    root.__path__ = []
+    sys.modules["nr3d_lib"] = root
     B.install_as_nr3d_lib_bindings()
-    # nr3d_lib/utils.py imports imageio / skimage / imagesize (not installable here); the files below take ONE helper from it
-    utils = types.ModuleType("nr3d_lib.utils")
-    utils.check_to_torch = lambda x, **kw: torch.as_tensor(x, **{k: v for k, v in kw.items() if k in ("dtype", "device")})
-    sys.modules["nr3d_lib.utils"] = utils
     yield B
     for k in [k for k in sys.modules if k == "nr3d_lib" or k.startswith("nr3d_lib.")]:
         del sys.modules[k]
@@ -45,34 +31,24 @@ def ref_tree():
 
 def test_reference_modules_import_over_the_shim(ref_tree):
     B = ref_tree
-    pack = importlib.import_module("nr3d_lib.graphics.pack_ops.pack_ops")
-    assert pack._backend is B._pack_ops
-    for k in pack.__all__:                                      # what `from .pack_ops import *` of the package __init__ would export
-        setattr(sys.modules["nr3d_lib.graphics.pack_ops"], k, getattr(pack, k))
-    march = importlib.import_module("nr3d_lib.graphics.raymarch.occgrid_raymarch")      # real package __init__ (dataclasses only) + the wrapper
-    assert march._backend is B._occ_grid
-    lotd = importlib.import_module("nr3d_lib.models.grid_encodings.lotd.lotd")
-    assert lotd._backend is B._lotd
-    sh = importlib.import_module("nr3d_lib.models.embedders.spherical_harmonics.sphere_harmonics")
-    assert sh._backend is B._shencoder
-    raytest = importlib.import_module("nr3d_lib.graphics.raytest")                     # imports _forest.raytrace_cuda_fixed at import time
-    assert callable(raytest.ray_box_intersection_fast_float_nocheck)
-    importlib.import_module("nr3d_lib.models.embedders.sinusoidal_cuda.freq")          # _freqencoder placeholder
-    importlib.import_module("nr3d_lib.models.grid_encodings.permuto.permuto")          # _permuto placeholder
+    built = {"nr3d_lib.bindings._pack_ops": B._pack_ops, "nr3d_lib.bindings._occ_grid": B._occ_grid, "nr3d_lib.bindings._lotd": B._lotd,
+             "nr3d_lib.bindings._shencoder": B._shencoder}
+    modules = {imp["module"] for imp in GOLDEN["imports"]}
+    assert set(built) <= modules and "nr3d_lib.bindings._forest" in modules
+    for imp in GOLDEN["imports"]:
+        mod = importlib.import_module(imp["module"])                      # `import nr3d_lib.bindings._x as _backend`
+        if imp["module"] in built:
+            assert mod is built[imp["module"]], imp
+        for name in imp["names"] or ():                                   # `from nr3d_lib.bindings._x import a, b` at import time
+            assert callable(getattr(mod, name)), imp
 
 
 def test_every_backend_name_the_reference_calls_exists(ref_tree):
     B = ref_tree
-    files = {"_pack_ops": ["graphics/pack_ops/pack_ops.py"], "_occ_grid": ["graphics/raymarch/occgrid_raymarch.py"],
-             "_lotd": ["models/grid_encodings/lotd/lotd.py", "models/grid_encodings/lotd/lotd_encoding.py", "models/grid_encodings/lotd/lotd_batched.py",
-                       "models/grid_encodings/lotd/lotd_forest.py"],
-             "_shencoder": ["models/embedders/spherical_harmonics/sphere_harmonics.py"]}
-    for mod, fs in files.items():
-        names = set()
-        for f in fs:
-            names |= set(re.findall(r"_backend\.(\w+)", open(os.path.join(REF, f)).read()))
+    assert set(GOLDEN["backend_calls"]) == {"_pack_ops", "_occ_grid", "_lotd", "_shencoder"}
+    for mod, names in GOLDEN["backend_calls"].items():
         shim = getattr(B, mod)
-        assert not [n for n in sorted(names) if not hasattr(shim, n)], mod
+        assert names and not [n for n in names if not hasattr(shim, n)], mod
 
 
 def test_placeholders_resolve_and_raise_on_use(ref_tree):
@@ -89,12 +65,15 @@ def test_placeholders_resolve_and_raise_on_use(ref_tree):
 
 
 def test_reference_lotd_module_builds_its_meta_through_the_shim(ref_tree):
-    """the reference's own `LoTD` nn.Module constructed on top of our `_lotd.LoDMeta` (host-side: no GPU needed): sizes as the oracle's"""
-    lotd = importlib.import_module("nr3d_lib.models.grid_encodings.lotd.lotd")
+    """the LoDMeta call the reference's own `LoTD` nn.Module makes (host-side: no GPU needed), replayed on the shim: sizes as the oracle's
+    and as the reference module derived them"""
     from oracle import lotd as olotd
-    res, feats, types_ = [8, 12, 18, 40, 64], [2] * 5, ["Dense", "Dense", "Dense", "Hash", "Hash"]
-    m = lotd.LoTD(3, res, feats, types_, hashmap_size=2 ** 12, dtype=torch.half, device=torch.device("cpu"))
-    om = olotd.LoDMeta(3, res, feats, types_, hashmap_size=2 ** 12)
-    assert m.n_params == om.n_params and list(m.level_n_feats) == feats
-    assert list(m.meta.level_offsets)[:len(res) + 1] == list(om.level_offsets)[:len(res) + 1]
-    assert m.out_features == 10 and m.in_features == 3
+    rec = GOLDEN["lotd_module"]
+    c = rec["cfg"]
+    assert rec["meta_args"] == [3, c["res"], c["feats"], c["types"], c["hashmap_size"], False]
+    m = importlib.import_module("nr3d_lib.bindings._lotd").LoDMeta(*rec["meta_args"])
+    om = olotd.LoDMeta(3, c["res"], c["feats"], c["types"], hashmap_size=c["hashmap_size"])
+    n_lvl = len(c["res"])
+    assert m.n_params == om.n_params == rec["n_params"] and m.level_n_feats == c["feats"] == rec["level_n_feats"]
+    assert m.level_offsets[:n_lvl + 1] == list(om.level_offsets)[:n_lvl + 1] == rec["level_offsets"][:n_lvl + 1]
+    assert sum(m.level_n_feats) == m.n_encoded_dims == rec["out_features"] == 10 and m.n_dims_to_encode == rec["in_features"] == 3
